@@ -65,7 +65,12 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the C3 / C4 sub-records")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float64), see dump_outputs()")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 # ---------------------------------------------------------------------------
@@ -381,6 +386,23 @@ def bind_to_gpu_numa_node(torch, local_rank):
     return None
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(torch, dirname, arrays):
+    """Writes the arrays a caller of the timed path receives as DIR/<name>.npy in float64, so that two builds can be
+    compared output for output (the inputs come from fixed seeds).  An array too long for DUMP_BYTES in all is
+    replaced by its values at fixed pseudo-random positions (seed 0), written beside it as DIR/<name>_rows.npy."""
+    os.makedirs(dirname, exist_ok=True)
+    cap = (DUMP_BYTES // len(arrays) - 1024) // 16           # worst case: every array sampled, values + positions
+    for name, t in arrays.items():
+        if t.numel() > cap:
+            rows = np.unique(np.random.default_rng(0).integers(0, t.numel(), cap))
+            np.save(os.path.join(dirname, f"{name}_rows.npy"), rows.astype(np.float64))
+            t = t[torch.from_numpy(rows).to(t.device)]
+        np.save(os.path.join(dirname, f"{name}.npy"), t.cpu().numpy().astype(np.float64))
+
+
 def run_b200(args, rank, local_rank, world):
     import torch
     import torch.distributed as dist
@@ -406,9 +428,10 @@ def run_b200(args, rank, local_rank, world):
 
     local_ev = []             # N > 1: CUDA events around every rank's own group()+reduce (the part before the merge)
 
-    def step():
+    def step(keep=False):
         # group(): RowIndex int32[n] + Groupby offsets int32[ng+1], both left in HBM behind the handle,
-        # and the SUM reducer, evaluated inside the same engine call
+        # and the SUM reducer, evaluated inside the same engine call.  keep: return the handle open
+        # (--dump-outputs reads it after the timed window)
         if world > 1 and profiling[0]:
             le0 = torch.cuda.Event(enable_timing=True); le0.record()
         gb = engine.Groupby([k], [0], _lib.NA_FIRST, reducers=[(_lib.OP_SUM, v)])
@@ -423,6 +446,8 @@ def run_b200(args, rank, local_rank, world):
             launches[0] += 2
             gkeys, sums = ddist.merge_partials_dense(gkeys, sums, _lib.OP_SUM, key_range=(0, G - 1))   # dictionary-coded keys
             launches[0] += ddist.LAST_MERGE_LAUNCHES
+        if keep:
+            return gb, gkeys if world > 1 else None, ng, sums
         gb.close()
         return None, None, ng, sums
 
@@ -445,8 +470,8 @@ def run_b200(args, rank, local_rank, world):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     ev0.record()
-    for _ in range(args.steps):
-        out = step()
+    for i in range(args.steps):
+        out = step(keep=args.dump_outputs is not None and i == args.steps - 1)
     ev1.record()
     barrier()
     ms_total = ev0.elapsed_time(ev1)
@@ -457,6 +482,14 @@ def run_b200(args, rank, local_rank, world):
     # that no step waited for them (the dense merge at N > 1 launches none of these families)
     own = ("col_stats", "radix_count", "radix_scatter", "group_offsets_from_counts", "group_offsets", "reduce_direct", "reduce")
     main_prof.extend(r for r in _lib.profile_records(reset=True) if r[0] in own)
+    if out[0] is not None:
+        if rank == 0:
+            arrays = {"row_index": out[0].order(), "group_offsets": out[0].offsets(), "group_sums": out[3]}
+            if world > 1:
+                arrays["group_keys"] = out[1]
+            dump_outputs(torch, args.dump_outputs, arrays)
+            del arrays
+        out[0].close()
     per_rank = None
     if world > 1:
         # every rank's own time in group()+reduce, so that the line shows how much of a step is the merge and

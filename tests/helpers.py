@@ -45,3 +45,35 @@ def assert_reducer_equal(got, want, op, vst, ctx=""):
     err = np.abs(g[~inf] - w[~inf])
     ok = err <= rtol * np.abs(w[~inf])
     assert np.all(ok), f"{ctx}: float mismatch, max rel err {np.max(err / np.maximum(np.abs(w[~inf]), 1e-300))}"
+
+
+def hook_inputs(name):
+    """The frames integration/check_hook.py ("group"), check_hook_reducers.py ("reducers") and check_hook_views.py
+    ("views") build, as numpy columns (same seeds and sizes)."""
+    if name == "group":
+        rng = np.random.default_rng(7)
+        n = 200_000
+        return {"k": rng.integers(0, 1000, n).astype(np.int32), "x": rng.standard_normal(n), "v": rng.random(n),
+                "idx": np.arange(n, dtype=np.int32)}
+    rng = np.random.default_rng(3 if name == "reducers" else 11)
+    n = 300_000 if name == "reducers" else 400_000
+    k = rng.integers(0, 5000, n).astype(np.int32)
+    v = rng.random(n); v[rng.random(n) < 0.05] = np.nan
+    w = rng.integers(-1000, 1000, n).astype(np.int16)
+    b = rng.random(n) < 0.3
+    cols = {"k": k, "v": v, "w": w, "b": b}
+    if name == "views":
+        cols["x"] = rng.integers(-2**60, 2**60, n)
+    return cols
+
+
+def digest(a):
+    """sha256 of a column's values (integers as int64, floats as float64 with one NaN pattern), for outputs too large
+    to store."""
+    import hashlib
+    a = np.asarray(a)
+    if a.dtype.kind == "f":
+        a = np.where(np.isnan(a), np.nan, a.astype(np.float64))
+    else:
+        a = a.astype(np.int64)
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()

@@ -320,6 +320,8 @@ def test_rows_beyond_2_pow_30():
     count + sum total on device-resident data, checked with engine kernels and cheap torch reductions."""
     import torch
     from datatable_b200 import engine
+    torch.cuda.empty_cache()                                  # what earlier tests left cached is free HBM too
+    engine.set_option("trim_scratch", 1)
     free, _ = torch.cuda.mem_get_info()
     n = 1_200_000_000
     if free < 80e9:
@@ -416,6 +418,8 @@ def test_group64_equals_group_and_crosses_int32():
         oh, fh, ngh = engine.group64(cols, [_lib.FLAG_SORT_ONLY] * len(sts), _lib.NA_LAST)      # host buffers, sort only
         ow, _, _ = engine.group(cols, [_lib.FLAG_SORT_ONLY] * len(sts), _lib.NA_LAST)
         assert fh is None and np.array_equal(oh, ow.astype(np.int64))
+    torch.cuda.empty_cache()                                  # what earlier tests left cached is free HBM too
+    engine.set_option("trim_scratch", 1)
     free, _ = torch.cuda.mem_get_info()
     n = 2**31 + 10_000_000
     if free < 130 * 2**30:
