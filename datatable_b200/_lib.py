@@ -18,6 +18,7 @@ NA_FIRST, NA_LAST, NA_REMOVE = 1, 2, 3
 OP_SUM, OP_MEAN, OP_MIN, OP_MAX, OP_COUNT, OP_COUNTNA, OP_NROWS = 1, 2, 3, 4, 5, 6, 7
 OP_FIRST, OP_LAST, OP_SD, OP_MEDIAN, OP_NUNIQUE = 8, 9, 10, 11, 12
 SET_UNION, SET_INTERSECT, SET_SETDIFF, SET_SYMDIFF = 0, 1, 2, 3
+WIN_CUMSUM, WIN_CUMPROD, WIN_CUMMIN, WIN_CUMMAX, WIN_CUMCOUNT, WIN_NGROUP, WIN_FILLNA, WIN_SHIFT = 1, 2, 3, 4, 5, 6, 7, 8
 OK, EINVAL, ENOTIMPL, ECUDA, ENOMEM, ENOSPACE = 0, -1, -2, -3, -4, -5
 
 EXPORTS = [
@@ -29,6 +30,7 @@ EXPORTS = [
     "dtb_profile_count", "dtb_profile_get", "dtb_profile_reset",
     "dtb_dense_scatter", "dtb_dense_compact",
     "dtb_sort_grouped", "dtb_set_select", "dtb_largest_group", "dtb_join", "dtb_cache_begin", "dtb_cache_end", "dtb_lower_bound",
+    "dtb_window_out_stype", "dtb_window",
 ]
 
 
@@ -123,6 +125,9 @@ def _load():
     lib.dtb_join.argtypes = [c.POINTER(dtb_col), c.POINTER(dtb_col), c.c_int, c.c_int64, c.c_int64, c.c_void_p,
                              c.c_void_p]
     lib.dtb_lower_bound.argtypes = [dtb_col, c.c_int64, dtb_col, c.c_int64, c.c_void_p, c.c_void_p]
+    lib.dtb_window_out_stype.argtypes = [c.c_int, c.c_int]
+    lib.dtb_window.argtypes = [c.c_int, c.c_int64, dtb_col, c.c_int64, c.c_void_p, c.c_void_p, c.c_int64, c.c_void_p,
+                               c.c_void_p]
     lib.dtb_memcpy.argtypes = [c.c_void_p, c.c_void_p, c.c_int64, c.c_void_p]
     lib.dtb_set_option.argtypes = [c.c_char_p, c.c_int64]
     lib.dtb_get_option.argtypes = [c.c_char_p, c.POINTER(c.c_int64)]

@@ -1354,6 +1354,63 @@ int dtb_gather(dtb_col src, int64_t nrows_src, const void* order, int order_is64
   return DTB_OK;
 }
 
+int dtb_window_out_stype(int op, int stype) { return window_out_stype_host(op, stype); }
+
+int dtb_window(int op, int64_t param, dtb_col value, int64_t nrows_value, const void* order, const void* offsets,
+               int64_t ngroups, dtb_stream stream, void* out)
+{
+  cudaStream_t s = (cudaStream_t)stream;
+  ArenaScope scope(s); if (scope.rc != DTB_OK) return scope.rc;
+  t_stats = dtb_call_stats{0, 0, 0, 0, 0};
+  if (op < DTB_WIN_CUMSUM || op > DTB_WIN_SHIFT) { set_error("unknown window op " + std::to_string(op)); return DTB_EINVAL; }
+  const bool uses_value = op != DTB_WIN_CUMCOUNT && op != DTB_WIN_NGROUP;
+  const int out_st = window_out_stype_host(op, value.stype);
+  if (!out_st) {
+    set_error("Invalid column of stype " + std::to_string(value.stype) + " in window op " + std::to_string(op));
+    return stype_supported(value.stype) ? DTB_EINVAL : DTB_ENOTIMPL;
+  }
+  if (op == DTB_WIN_SHIFT && (param < INT32_MIN || param > INT32_MAX)) {
+    set_error("Value is too large to fit in an int32"); return DTB_EINVAL;
+  }
+  if (ngroups < 0 || nrows_value < 0) { set_error("negative size"); return DTB_EINVAL; }
+  if (!offsets) { set_error("offsets is NULL"); return DTB_EINVAL; }
+  if (uses_value && !value.data && nrows_value > 0) { set_error("value column data is NULL"); return DTB_EINVAL; }
+  DTB_TRY(ensure_context());
+  if (ngroups == 0) return DTB_OK;
+
+  DevIn d_off; DTB_TRY(d_off.bind(offsets, sizeof(int32_t) * (size_t)(ngroups + 1), s));
+  // caller-supplied offsets must be a Groupby: offsets[0] = 0, strictly increasing (groupby.h:41-47)
+  int32_t n32 = 0;
+  int bad = 0;
+  {
+    DevBuf d_bad; DTB_TRY(d_bad.alloc(sizeof(int), s));
+    DTB_CUDA_CHECK(cudaMemsetAsync(d_bad.p, 0, sizeof(int), s));
+    DTB_TRY(launch_offsets_check((const int32_t*)d_off.dptr, ngroups, d_bad.as<int>(), s));
+    DTB_CUDA_CHECK(cudaMemcpyAsync(&n32, (const int32_t*)d_off.dptr + ngroups, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    DTB_CUDA_CHECK(cudaMemcpyAsync(&bad, d_bad.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+    DTB_CUDA_CHECK(cudaStreamSynchronize(s));
+  }
+  if (bad) {
+    set_error("offsets is not a Groupby: offsets[0] must be 0 and offsets strictly increasing (group " +
+              std::to_string(bad - 1) + " is empty or out of order)");
+    return DTB_EINVAL;
+  }
+  const int64_t n = n32;
+  if (!out && n > 0) { set_error("out is NULL"); return DTB_EINVAL; }
+  DevIn d_val, d_ord;
+  if (uses_value) DTB_TRY(d_val.bind(value.data, (size_t)nrows_value * stype_bytes(value.stype), s));
+  DTB_TRY(d_ord.bind(order, (size_t)n * sizeof(int32_t), s));
+  DevOut d_out; DTB_TRY(d_out.bind(out, (size_t)n * stype_bytes(out_st), s));
+  DevBuf scratch; DTB_TRY(scratch.alloc(window_scratch_bytes(n), s));
+  DTB_TRY(launch_window(op, param, d_val.dptr, value.stype, uses_value ? nrows_value : 0, (const int32_t*)d_ord.dptr,
+                        (const int32_t*)d_off.dptr, ngroups, n, d_out.dptr, scratch.p, s));
+  if (d_out.staged()) {
+    DTB_TRY(d_out.finish((size_t)n * stype_bytes(out_st), s));
+    DTB_CUDA_CHECK(cudaStreamSynchronize(s));
+  }
+  return DTB_OK;
+}
+
 int dtb_dense_scatter(const void* keys, int key_stype, const void* vals, int64_t n, int64_t kmin, int64_t table_size,
                       void* table, void* present, dtb_stream stream)
 {

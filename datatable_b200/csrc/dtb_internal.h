@@ -217,6 +217,12 @@ void fill_u64(unsigned long long* p, int64_t n, unsigned long long v, cudaStream
 int launch_gather(const void* src, int stype, int64_t nrows_src, const void* order,
                   int order_is64, int64_t n, void* out, cudaStream_t s);
 
+// grouped cumulative / window functions (dtb_window.cu); scratch: window_scratch_bytes(n) of device memory
+int window_out_stype_host(int op, int stype);
+size_t window_scratch_bytes(int64_t n);
+int launch_window(int op, int64_t param, const void* value, int stype, int64_t nrows_value, const int32_t* order,
+                  const int32_t* offsets, int64_t ngroups, int64_t n, void* out, void* scratch, cudaStream_t s);
+
 int launch_iota32(int32_t* out, int64_t n, cudaStream_t s);
 int launch_widen_u32(const uint32_t* in, int64_t n, int64_t* out, cudaStream_t s);   // ARR32 bit patterns -> ARR64
 

@@ -15,7 +15,7 @@ import ctypes
 import numpy as np
 
 from . import _lib
-from ._lib import (BOOL, INT8, INT16, INT32, INT64, FLOAT32, FLOAT64, FLAG_DESCENDING,
+from ._lib import (BOOL, INT8, INT16, INT32, INT64, FLOAT32, FLOAT64, DATE32, TIME64, FLAG_DESCENDING,
                    FLAG_SORT_ONLY, NA_FIRST, NA_LAST, NA_REMOVE, check, dtb_col, lib)
 
 try:  # torch is plumbing only: device memory + streams
@@ -27,12 +27,13 @@ _NP2ST = {np.dtype(np.bool_): BOOL, np.dtype(np.int8): INT8, np.dtype(np.int16):
           np.dtype(np.int32): INT32, np.dtype(np.int64): INT64,
           np.dtype(np.float32): FLOAT32, np.dtype(np.float64): FLOAT64}
 _ST2NP = {BOOL: np.int8, INT8: np.int8, INT16: np.int16, INT32: np.int32, INT64: np.int64,
-          FLOAT32: np.float32, FLOAT64: np.float64}
+          FLOAT32: np.float32, FLOAT64: np.float64, DATE32: np.int32, TIME64: np.int64}
 
 
 def _torch_dtype(st):
     return {BOOL: torch.int8, INT8: torch.int8, INT16: torch.int16, INT32: torch.int32,
-            INT64: torch.int64, FLOAT32: torch.float32, FLOAT64: torch.float64}[st]
+            INT64: torch.int64, FLOAT32: torch.float32, FLOAT64: torch.float64, DATE32: torch.int32,
+            TIME64: torch.int64}[st]
 
 
 def is_tensor(x):
@@ -262,6 +263,10 @@ class Groupby:
                              self.ngroups, _stream(), ctypes.c_void_p(optr)))
         return out
 
+    def window(self, op, value, param=0):
+        """Window function over the handle's RowIndex and Groupby (CUDA tensor, one value per row of the RowIndex)."""
+        return window(op, value, self.order_col(), self.offsets_col(), param)
+
     def order_col(self):
         """The RowIndex as a zero-copy column view (valid while the handle lives)."""
         return Col.from_ptr(self.order_ptr, INT32, self.norder, owner=self)
@@ -331,6 +336,49 @@ def reduce(op, value, order, offsets, stype=None):
                          ctypes.c_void_p(o.ptr) if o is not None else None, is64,
                          ctypes.c_void_p(f.ptr), ngroups, _stream(), ctypes.c_void_p(optr)))
     return out
+
+
+def window_out_stype(op, stype):
+    return lib.dtb_window_out_stype(op, stype)
+
+
+def window(op, value, order, offsets, param=0, stype=None):
+    """Grouped cumulative / window function (dtb_window): one value per position of the grouped frame given by
+    RowIndex `order` (None = identity) and Groupby `offsets`.  param: `reverse` for WIN_CUMSUM .. WIN_FILLNA, the
+    shift n for WIN_SHIFT.  `value` is ignored (may be None) for WIN_CUMCOUNT / WIN_NGROUP.  The result lives where
+    the value column (or, without one, the offsets) lives."""
+    f = Col(offsets)
+    ngroups = f.nrows - 1
+    if op in (_lib.WIN_CUMCOUNT, _lib.WIN_NGROUP):
+        vst, vptr, vn, device = INT8, 0, 0, f.on_device
+    else:
+        v = Col(value, stype)
+        vst, vptr, vn, device = v.stype, v.ptr, v.nrows, v.on_device
+    out_st = lib.dtb_window_out_stype(op, vst)
+    if not out_st:
+        raise _lib.DtbValueError(f"Invalid column of stype {vst} in window op {op}")
+    o = None if order is None else Col(order)
+    if o is not None and o.stype != INT32:
+        raise _lib.DtbValueError("order must be int32")
+    if ngroups <= 0:
+        n = 0
+    elif isinstance(offsets, Col):
+        n = _offsets_total(f)
+    else:
+        last = offsets[-1]
+        n = int(last.item() if is_tensor(last) else last)
+    out, optr = _alloc(n, out_st, device)
+    check(lib.dtb_window(op, int(param), dtb_col(ctypes.c_void_p(vptr), vst, 0), vn,
+                         ctypes.c_void_p(o.ptr) if o is not None else None, ctypes.c_void_p(f.ptr), ngroups,
+                         _stream(), ctypes.c_void_p(optr)))
+    return out
+
+
+def _offsets_total(f):
+    """offsets[ngroups] of an offsets column given as a Col (e.g. the HBM-resident offsets of a Groupby handle)."""
+    n = ctypes.c_int32(0)
+    check(lib.dtb_memcpy(ctypes.byref(n), ctypes.c_void_p(f.ptr + 4 * (f.nrows - 1)), 4, _stream()))
+    return n.value
 
 
 def gather(src, order, stype=None):

@@ -9,6 +9,7 @@ no general expression engine (SURVEY.md 8: out of scope).
     f.A, f["A"], -f.A        src/datatable/expr/                               f / ColRef
     by(...), sort(...)       src/core/expr/py_by.cc, py_sort.cc:40-110         by / sort
     dt.sum/mean/min/max/count  src/datatable/expr/reduce.py:49-153             sum_/mean/min_/max_/count
+    dt.cumsum/.../shift/fillna  src/core/expr/fexpr_cumsumprod.cc, ...        cumsum .. fillna (Window)
     DT[i, j, by, sort]       src/core/frame/__getitem__.cc:47-194,
                              src/core/expr/eval_context.cc:144-288, 473-520    Frame.__getitem__
 
@@ -20,7 +21,7 @@ through the RowIndex; group keys are the first row of every group
 import numpy as np
 
 from . import _lib, engine
-from ._lib import (BOOL, INT8, INT16, INT32, INT64, FLOAT32, FLOAT64, FLAG_DESCENDING,
+from ._lib import (BOOL, INT8, INT16, INT32, INT64, FLOAT32, FLOAT64, DATE32, TIME64, FLAG_DESCENDING,
                    FLAG_SORT_ONLY, NA_FIRST, NA_LAST, NA_REMOVE)
 
 try:
@@ -29,7 +30,7 @@ except Exception:  # pragma: no cover
     torch = None
 
 _NA_POS = {"first": NA_FIRST, "last": NA_LAST, "remove": NA_REMOVE}
-_NA_VALUE = {INT8: -2**7, INT16: -2**15, INT32: -2**31, INT64: -2**63, BOOL: -128}
+_NA_VALUE = {INT8: -2**7, INT16: -2**15, INT32: -2**31, INT64: -2**63, BOOL: -128, DATE32: -2**31, TIME64: -2**63}
 
 
 # ---------------------------------------------------------------------------
@@ -80,6 +81,52 @@ def nunique(x): return Reducer(_lib.OP_NUNIQUE, "nunique", x) if isinstance(x, (
 
 def count(x=None):
     return Reducer(_lib.OP_NROWS if x is None else _lib.OP_COUNT, "count", x)
+
+
+class Window:
+    """A grouped cumulative / window function: one value per row of its group (the reference's GtoALL columns)."""
+
+    def __init__(self, op, name, arg, param=0):
+        self.op, self.opname, self.arg, self.param = op, name, arg, param
+
+    def __repr__(self):
+        if self.op == _lib.WIN_SHIFT:
+            return f"shift({self.arg!r}, n={self.param})"
+        arg = "" if self.arg is None else f"{self.arg!r}, "
+        return f"{self.opname}({arg}reverse={bool(self.param)})"
+
+
+def _window(op, name, x, param):
+    if isinstance(x, (list, tuple)):                 # cumsum([f.a, f.b]): one column per argument
+        return [Window(op, name, _as_ref(a), param) for a in _flatten(x)]
+    return Window(op, name, _as_ref(x), param)
+
+
+# grouped cumulative functions (column/cumsumprod.h, cumminmax.h, cumcountngroup.h) and shift / fillna
+# (expr/head_func_shift.cc, fexpr_fillna.cc); under by() they restart in every group
+def cumsum(x, reverse=False): return _window(_lib.WIN_CUMSUM, "cumsum", x, int(bool(reverse)))
+def cumprod(x, reverse=False): return _window(_lib.WIN_CUMPROD, "cumprod", x, int(bool(reverse)))
+def cummin(x, reverse=False): return _window(_lib.WIN_CUMMIN, "cummin", x, int(bool(reverse)))
+def cummax(x, reverse=False): return _window(_lib.WIN_CUMMAX, "cummax", x, int(bool(reverse)))
+def cumcount(reverse=False): return Window(_lib.WIN_CUMCOUNT, "cumcount", None, int(bool(reverse)))
+def ngroup(reverse=False): return Window(_lib.WIN_NGROUP, "ngroup", None, int(bool(reverse)))
+
+
+def shift(x, n=1):
+    """Value n rows earlier in the group (n < 0: later), NA where that row is outside the group."""
+    if not isinstance(n, int) or isinstance(n, bool):
+        raise TypeError(f"Argument n in shift() should be an integer, instead got {type(n)}")
+    if not -2**31 <= n < 2**31:
+        raise ValueError(f"Value is too large to fit in an int32: {n}")
+    return Window(_lib.WIN_SHIFT, "shift", _as_ref(x), n)
+
+
+def fillna(x, value=None, reverse=False):
+    """Forward fill inside the group (backward with reverse=True).  Filling with a value is elementwise and not on
+    the GPU path."""
+    if value is not None:
+        raise NotImplementedError("fillna(value=...) is an elementwise expression, outside the GPU hot path")
+    return _window(_lib.WIN_FILLNA, "fillna", x, int(bool(reverse)))
 
 
 class by:
@@ -397,7 +444,10 @@ def _evaluate(DT, j, by_, sort_, isel=None):
         if m is not None:
             needed += [r.name for r in m.cols]
     for e in exprs:
-        nm = e.arg.name if isinstance(e, Reducer) and e.arg is not None else getattr(e, "name", None)
+        if isinstance(e, (Reducer, Window)):
+            nm = None if e.arg is None else e.arg.name
+        else:
+            nm = e.name
         if nm is not None:
             needed.append(nm)
     copy_stream = None
@@ -463,6 +513,15 @@ def _evaluate(DT, j, by_, sort_, isel=None):
     ngroups = None
     gb = None
     has_reducer = any(isinstance(e, Reducer) for e in exprs)
+    # GtoALL (eval_context.cc:144-172): one output row per row of the grouped frame -- j holds a window function, or a
+    # plain column next to a reducer under by(); reducers are then repeated on every row of their group
+    gtoall = any(isinstance(e, Window) for e in exprs) or (
+        by_ is not None and has_reducer and any(isinstance(e, ColRef) for e in exprs))
+    for e in exprs:
+        if isinstance(e, Window) and e.arg is not None:
+            st_ = DT._col(e.arg.name).stype
+            if not engine.window_out_stype(e.op, st_):
+                raise TypeError(f"Invalid column of type {_STYPE_NAME.get(st_, st_)} in {e!r}")
     sliced = False
     if keycols and isel is not None:
         # i under by() / sort(): group() first, then the slice inside every group; its positions are composed with
@@ -493,7 +552,7 @@ def _evaluate(DT, j, by_, sort_, isel=None):
             rng_ = range(*isel.indices(n_))
         order = torch.arange(rng_.start, rng_.stop, rng_.step, dtype=torch.int32, device="cuda")
     elif keycols:
-        if by_ is not None and has_reducer:
+        if by_ is not None and has_reducer and not gtoall:
             # RowIndex + Groupby stay in HBM behind a handle; reducers go through it
             # the reducers of j are known before group() runs: hand them over so that the engine can
             # overlap them with the sort (dtb_groupby_create_reduce)
@@ -548,6 +607,14 @@ def _evaluate(DT, j, by_, sort_, isel=None):
             data = data.cpu().numpy()
         out._cols[name] = data
         out._stypes[name] = st
+
+    if gtoall:
+        if offsets is None:                     # no by(): one group over the rows kept (Groupby::single_group)
+            n_ = DT.nrows if order is None else len(order)
+            offsets = torch.tensor([0, n_] if n_ else [0], dtype=torch.int32, device="cuda")
+        _evaluate_gtoall(by_, names, exprs, dcol, add, order, offsets)
+        out._nrows = DT.nrows if order is None else len(order)
+        return out
 
     if by_ is not None:
         if has_reducer and sliced:
@@ -625,6 +692,52 @@ def _evaluate(DT, j, by_, sort_, isel=None):
     return out
 
 
+def _evaluate_gtoall(by_, names, exprs, dcol, add, order, offsets):
+    """j evaluated per row of the grouped frame (RowIndex `order`, None = identity; Groupby `offsets`): by-columns
+    and plain columns gathered through the RowIndex, window functions from dtb_window, reducers computed per group
+    and repeated on every row of the group (gathered through the group id of every row)."""
+    def rows(c):
+        return c.data if order is None else engine.gather(c, order)
+    bynames = [] if by_ is None else [ref.name for ref in by_.cols]
+    final = _unique_names(bynames + list(names))
+    for ref, name in zip(by_.cols if by_ is not None else [], final):
+        c = dcol(ref.name)
+        add(name, rows(c), c.stype)
+    gid = None
+    for name, e in zip(final[len(bynames):], exprs):
+        if isinstance(e, Window):
+            c = None if e.arg is None else dcol(e.arg.name)
+            st = engine.window_out_stype(e.op, INT8 if c is None else c.stype)
+            add(name, engine.window(e.op, c, order, offsets, e.param), st)
+        elif isinstance(e, Reducer):
+            if gid is None:
+                gid = engine.window(_lib.WIN_NGROUP, None, None, offsets)
+            st = _red_stype(dcol, e)
+            add(name, engine.gather(engine.Col(_reduce(dcol, e, order, offsets), st), gid), st)
+        else:
+            c = dcol(e.name)
+            add(name, rows(c), c.stype)
+
+
+def _unique_names(names):
+    """Duplicate column names made unique the way the reference's Frame does it: a name that ends in digits counts
+    on from them ("x9" -> "x10"), any other name gets ".0", ".1", ... ("v" -> "v.0")."""
+    out, seen = [], set()
+    for name in names:
+        if name in seen:
+            stem = name.rstrip("0123456789")
+            if stem != name:
+                k = int(name[len(stem):]) + 1
+            else:
+                stem, k = (stem if stem.endswith(".") else stem + "."), 0
+            while f"{stem}{k}" in seen:
+                k += 1
+            name = f"{stem}{k}"
+        seen.add(name)
+        out.append(name)
+    return out
+
+
 def j_is_all(j):
     return isinstance(j, slice) and j == slice(None)
 
@@ -635,20 +748,27 @@ def _resolve_j(DT, j):
     if isinstance(j, dict):
         return list(j.keys()), [_as_expr(v) for v in j.values()]
     if isinstance(j, (list, tuple)):
-        es = [_as_expr(v) for v in j]
+        es = [_as_expr(v) for v in _flatten(j)]
     else:
         es = [_as_expr(j)]
     names = []
+    unnamed = 0
     for e in es:
         if isinstance(e, Reducer):
             names.append("count" if e.arg is None else e.arg.name)     # reducers keep the column's name
+        elif isinstance(e, Window):
+            if e.arg is None:                                           # cumcount / ngroup: C0, C1, ...
+                names.append(f"C{unnamed}")
+                unnamed += 1
+            else:
+                names.append(e.arg.name)
         else:
             names.append(e.name)
     return names, es
 
 
 def _as_expr(v):
-    if isinstance(v, (Reducer, ColRef)):
+    if isinstance(v, (Reducer, ColRef, Window)):
         return v
     if isinstance(v, str):
         return ColRef(v)
@@ -668,6 +788,8 @@ def _red_stype(dcol, e):
 
 
 _SORTED_OPS = (_lib.OP_MEDIAN, _lib.OP_NUNIQUE)
+_STYPE_NAME = {BOOL: "bool8", INT8: "int8", INT16: "int16", INT32: "int32", INT64: "int64", FLOAT32: "float32",
+               FLOAT64: "float64", DATE32: "date32", TIME64: "time64"}
 
 
 def _reduce(dcol, e, order, offsets):

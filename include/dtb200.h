@@ -249,6 +249,39 @@ DTB_API int dtb_gather(dtb_col src, int64_t nrows_src,
                dtb_stream stream, void* out);
 
 /*
+ * dtb_window -- grouped cumulative and window functions: one output row per position of the grouped frame, in
+ * group order.  Replaces the materialisation of the reference's per-row group functions (the GtoALL columns of
+ * EvalContext):
+ */
+#define DTB_WIN_CUMSUM   1   /* CumSumProd_ColumnImpl<T,true,REV>      column/cumsumprod.h:48-95     */
+#define DTB_WIN_CUMPROD  2   /* CumSumProd_ColumnImpl<T,false,REV>                                   */
+#define DTB_WIN_CUMMIN   3   /* CumMinMax_ColumnImpl<T,true,REV>       column/cumminmax.h:48-110     */
+#define DTB_WIN_CUMMAX   4
+#define DTB_WIN_CUMCOUNT 5   /* CumcountNgroup_ColumnImpl<true,REV>    column/cumcountngroup.h:52-70 */
+#define DTB_WIN_NGROUP   6
+#define DTB_WIN_FILLNA   7   /* FExpr_FillNA::fill_rowindex            expr/fexpr_fillna.cc:86-118   */
+#define DTB_WIN_SHIFT    8   /* compute_lag_rowindex                   expr/head_func_shift.cc:41-62 */
+/*
+ * Output stype of window op `op` over a value column of `stype`; 0 = invalid combination (TypeError in the
+ * reference: cumsum / cumprod of date32 or time64).  cumsum / cumprod: bool, int8..int64 -> int64 (wraps mod 2^64),
+ * float32 / float64 unchanged.  cummin / cummax / fillna / shift keep the stype.  cumcount / ngroup: int64.
+ */
+DTB_API int dtb_window_out_stype(int op, int stype);
+/*
+ *   value, nrows_value : the value column (ignored by CUMCOUNT / NGROUP), viewed through `order`
+ *   order              : int32[offsets[ngroups]] RowIndex, or NULL = identity
+ *   offsets            : int32[ngroups+1] Groupby (one group [0, n] for a frame without by())
+ *   param              : `reverse` (0 / 1) for CUMSUM .. FILLNA; the shift n for SHIFT (int32 range, else
+ *                        DTB_EINVAL): out[p] = v[order[p - n]] when p - n lies in p's group, else NA
+ *   out                : offsets[ngroups] elements of dtb_window_out_stype(op, value.stype)
+ * NA counts as 0 in CUMSUM and 1 in CUMPROD; CUMMIN / CUMMAX / FILLNA skip NAs (a leading NA stays NA) and break
+ * ties toward the current row.  Integer sums and products are exact mod 2^64; float sums and products are
+ * accumulated in float64 with an unspecified association order.  Everything else is bit-exact.
+ */
+DTB_API int dtb_window(int op, int64_t param, dtb_col value, int64_t nrows_value,
+               const void* order, const void* offsets, int64_t ngroups, dtb_stream stream, void* out);
+
+/*
  * dtb_slice_groups -- the `i` node of DT[i, j, by(), sort()] when i is an integer slice (or an integer: the
  * slice [i, i+1)); replaces FExpr_Literal_SliceInt::evaluate_iby (expr/fexpr_literal_sliceint.cc:82-170) and
  * FExpr_Literal_Int::evaluate_iby (expr/fexpr_literal_int.cc:146-192): the slice is applied inside every group
